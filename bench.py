@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- Mrays/s of the NeuMan ray-marching hot path at 128+128 samples on N B200s.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 Workload (config.workload): render_vanilla -- background NeRF, 1280x720 = 921 600 rays, 128 coarse +
 128 importance samples (the fine net evaluates 256), seeded default-init weights, synthetic camera:
@@ -15,6 +15,10 @@ fixed, so scaling is "strong".
             frame copied device->host inside the timed region.
 `roofline`: the dominant kernel (k_mlp_tc, tcgen05 fp16xfp16->fp32) timed per launch with CUDA events on
             its own stream inside the timed region (nm_profile_*), algorithmic FLOPs = evals x 1 186 816.
+`--dump-outputs DIR`: after the timed steps, the frame the last timed step computed -- what the device-resident call
+            hands back -- is written as DIR/rgb.npy (float32 [921600, 3]) and DIR/depth.npy (float32 [921600]), 14.7 MB
+            in all.  Weights and camera are seeded, so the same arguments give the same inputs on every run and two
+            builds can be compared output for output.
 `configs` : BASELINE.json configs 2-5 at their stated sizes (device-resident, 1 warm + 2 timed frames each):
             Mrays/s, MLP evaluations, hit rays, MLP TFLOP/s.
 `cpu_baseline` / `--impl reference`: the UNMODIFIED reference's own render_vanilla (baseline/_ref, installed by
@@ -213,7 +217,10 @@ def main():
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-configs", action="store_true", help="skip the cfg2-5 side measurements")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's rgb / depth as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be >= 1")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local = int(os.environ.get("LOCAL_RANK", "0"))
@@ -300,6 +307,10 @@ def main():
     clocks = sampler.stop() if sampler else None
     ms_step = ms_total / args.steps
     value = n_pix / (ms_step * 1e3)
+    if args.dump_outputs and rank == 0:
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, t in (("rgb", frame[0]), ("depth", frame[1])):
+            np.save(os.path.join(args.dump_outputs, f"{name}.npy"), t.float().cpu().numpy())
     for _ in range(2):
         step_e2e()
     ms_e2e, host = timed(step_e2e, args.steps)

@@ -33,62 +33,54 @@ def test_state_dict_layout_matches_reference_names():
     assert h.coarse_human_net.pos_pe.mapping == "rotate" and h.coarse_bkg_net.pos_pe.mapping == "posenc"
 
 
-@pytest.mark.reference
 def test_state_dict_keys_equal_reference():
-    from oracle import ref_import, ref_opts, scenes
-    ref = ref_import.load()
-    rc, rf = scenes.seed_nets(ref.vanilla.build_nerf, ref_opts.default_opt(), 1)
+    """The seeded background nets have the reference's keys, shapes and default-init values (tests/golden/reference.npz)."""
+    from oracle import scenes
+    from tests import util
+    g = util.golden("reference.npz")
     pc, pf = scenes.seed_nets(nb.build_nerf, nb.default_opt(use_cuda=False), 1)
-    for a, b in ((rc, pc), (rf, pf)):
-        sa, sb = a.state_dict(), b.state_dict()
-        assert list(sa) == list(sb)
-        for k in sa:
-            assert torch.equal(sa[k], sb[k]), k
-    pc.load_state_dict(rc.state_dict())                              # checkpoints load unchanged
+    util.assert_state_dict_is_the_references(pc.state_dict(), g, "bsd_coarse")
+    util.assert_state_dict_is_the_references(pf.state_dict(), g, "bsd_fine")
 
 
-@pytest.mark.reference
 @pytest.mark.parametrize("scale_type", ["linear", "tanh", "no"])
 def test_offset_net_equals_reference(scale_type):
     """neuman_b200.OffsetNet (library-GEMM forward, models/vanilla.py:169-205) against the reference's OffsetNet with the
-    same seeded weights: bit-equal on the CPU, gradients included."""
-    from oracle import ref_import
-    ref = ref_import.load()
+    same seeded weights (tests/golden/reference.npz): bit-equal on the CPU, gradients included (sampled)."""
+    from tests import util
+    g = util.golden("reference.npz")
     opt = nb.default_opt(use_cuda=False, num_offset_nets=1, offset_scale=0.7, offset_scale_type=scale_type)
     torch.manual_seed(3)
     mine = nb.build_offset_net(opt)
-    torch.manual_seed(3)
-    theirs = ref.vanilla.build_offset_net(opt)
-    assert list(mine.state_dict()) == list(theirs.state_dict())
-    theirs.load_state_dict(mine.state_dict())
-    x = torch.randn(40, 6, 4)
-    a, b = mine(x), theirs(x)
-    assert a.shape == (40, 6, 3) and torch.equal(a, b)
+    assert list(mine.state_dict()) == [str(k) for k in g[f"off_{scale_type}_sd_keys"]]
+    assert [k for k, _ in mine.named_parameters()] == [str(k) for k in g[f"off_{scale_type}_keys"]]
+    x = torch.from_numpy(g[f"off_{scale_type}_x"])
+    a = mine(x)
+    assert a.shape == (40, 6, 3) and torch.equal(a, torch.from_numpy(g[f"off_{scale_type}_y"]))
     a.square().sum().backward()
-    b.square().sum().backward()
-    for (k, p), q in zip(mine.named_parameters(), theirs.parameters()):
-        assert torch.allclose(p.grad, q.grad, rtol=1e-5, atol=1e-7), k
+    for i, (k, p) in enumerate(mine.named_parameters()):
+        idx = util.pick(p.grad.numel(), g[f"off_{scale_type}_grads"].shape[1], 200 + i)
+        q = torch.from_numpy(g[f"off_{scale_type}_grads"][i, :len(idx)])
+        assert torch.allclose(p.grad.reshape(-1)[torch.from_numpy(idx)], q, rtol=1e-5, atol=1e-7), k
+        assert abs(p.grad.double().norm().item() - g[f"off_{scale_type}_norms"][i]) <= 1e-5 * g[f"off_{scale_type}_norms"][i] + 1e-7, k
 
 
-@pytest.mark.reference
 @pytest.mark.parametrize("posenc", ["posenc", "rotate"])
 def test_module_interface_layer_by_layer_equals_reference(posenc):
     """SURVEY.md 8b lists Embedder.forward and NeRF.forward among the signatures to preserve: the mirrors evaluate them with
     library ops (the fused kernels serve Joiner.forward); bit-equal to the reference's modules on the CPU, and
-    NeRF(Embedder(x), Embedder(v)) == the reference's Joiner."""
-    from oracle import ref_import, ref_opts
-    ref = ref_import.load()
+    NeRF(Embedder(x), Embedder(v)) == the reference's Joiner (tests/golden/reference.npz)."""
+    from oracle import scenes
+    from tests import util
+    g = {k[len(f"mi_{posenc}_"):]: v for k, v in util.golden("reference.npz").items() if k.startswith(f"mi_{posenc}_")}
     torch.manual_seed(2)
     mine, _ = nb.build_nerf(nb.default_opt(use_cuda=False, posenc=posenc))
-    torch.manual_seed(2)
-    theirs, _ = ref.vanilla.build_nerf(ref_opts.default_opt(posenc=posenc))
-    for pe in (theirs.pos_pe, theirs.dir_pe):
-        if hasattr(pe, "bvals"):
-            pe.bvals = pe.bvals.cpu()                # the reference parks them on the GPU whenever one is visible
-    x, v = torch.randn(7, 5, 3), torch.randn(7, 5, 3)
+    assert abs(scenes.net_checksum(mine) - g["sum"]) <= 1e-9 * g["sum"]
+    x, v = torch.from_numpy(g["x"]), torch.from_numpy(g["v"])
     e, d = mine.pos_pe(x), mine.dir_pe(v)
-    assert torch.equal(e, theirs.pos_pe(x)) and torch.equal(d, theirs.dir_pe(v)) and e.shape[-1] == 63 and d.shape[-1] == 27
-    assert torch.equal(mine.nerf(e, d), theirs(x, v))
+    assert torch.equal(e, torch.from_numpy(g["pos"])) and torch.equal(d, torch.from_numpy(g["dir"]))
+    assert e.shape[-1] == 63 and d.shape[-1] == 27
+    assert torch.equal(mine.nerf(e, d), torch.from_numpy(g["out"]))
 
 
 def test_offset_net_joiner_form_stays_on_the_modules_device():

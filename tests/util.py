@@ -13,6 +13,27 @@ def golden(name):
     return dict(np.load(os.path.join(GOLD, name)))
 
 
+def pick(n, k, seed):
+    """k seeded positions in [0, n) (all of them when n <= k), sorted: where a golden fixture samples a large array."""
+    if n <= k:
+        return np.arange(n)
+    return np.sort(np.random.RandomState(seed).choice(n, k, replace=False))
+
+
+def assert_state_dict_is_the_references(sd, G, prefix):
+    """`sd` has the keys in the same order, the same shapes, and the same values: float64 sums and the
+    values at the seeded positions the fixture `G` sampled (tools/make_golden_reference.py: state_digest)."""
+    keys = [str(k) for k in G[f"{prefix}_keys"]]
+    assert list(sd) == keys
+    for i, k in enumerate(keys):
+        v = sd[k].detach().cpu()
+        assert "x".join(map(str, v.shape)) == str(G[f"{prefix}_shapes"][i]), k
+        sums = np.array([v.double().sum().item(), v.double().abs().sum().item()])
+        assert np.allclose(sums, G[f"{prefix}_sums"][i], rtol=1e-12, atol=1e-12), k
+        idx = pick(v.numel(), G[f"{prefix}_vals"].shape[1], i)
+        assert np.array_equal(v.reshape(-1)[torch.from_numpy(idx)].numpy(), G[f"{prefix}_vals"][i, :len(idx)]), k
+
+
 def product_nets(device="cpu"):
     """(coarse, fine, human) seeded exactly like tools/make_golden.py."""
     import neuman_b200 as nb
